@@ -56,6 +56,23 @@ def n_systems(data):
     return int(data[S.n_atoms].shape[0])
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write the outputs of the last timed step as ``out_dir/<name>.npy`` (fp32 as computed, fp64 kept), so that two
+    builds run with the same arguments -- hence the same seeded inputs and weights -- can be compared output for output.
+    Should they exceed 64 MB together, every array keeps a fixed, seeded sample of its rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT and a.ndim > 0:
+            keep = max(1, int(a.shape[0] * DUMP_LIMIT // total))
+            a = a[np.sort(np.random.RandomState(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------- algorithmic bytes
 def edge_kernel_bytes(E, N, F, has_mu, backward):
     """SURVEY.md §8(d) 'no-reuse gather model' per launch of the fused PaiNN edge kernel.
@@ -475,6 +492,8 @@ def run_cuda(args, rank, world, local_rank):
                 kernel_ms[kind] += [(a.elapsed_time(b), hm) for a, b, hm in pairs[kind]]
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: out[k].detach().cpu().numpy() for k in model.model_outputs if k in out})
     launches = launches_per_step * args.steps if use_graph else _lib.launch_count - launches0
     timing["on"] = False
     if not use_graph:
@@ -653,7 +672,7 @@ def run_cuda(args, rank, world, local_rank):
 
 
 # ------------------------------------------------------------------------------------------------- spatial (cfg5) arm
-def run_spatial(args, rank, world, local_rank, steps=None, warmup=None, cpu_leg=True):
+def run_spatial(args, rank, world, local_rank, steps=None, warmup=None, cpu_leg=True, dump_dir=None):
     """cfg5: ONE periodic box (default 262144 atoms, PaiNN 128x3, E+F) cut into `world` slabs; every rank owns a slab, holds
     read-only ghost rows of the senders it does not own, and exchanges (x, mu) ghost rows per interaction block over NCCL
     point-to-point (gradients back in the reverse sweep).  STRONG scaling: the box is fixed, `value` = whole-box evaluations
@@ -786,6 +805,8 @@ def run_spatial(args, rank, world, local_rank, steps=None, warmup=None, cpu_leg=
         step_ev.append((s_, e_))
     torch.cuda.synchronize()
     timing["on"] = False
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"energy": energy.detach().cpu().numpy(), "forces": forces.detach().cpu().numpy()})
     launches = _lib.launch_count - c0
     clocks = sampler.stop() if sampler is not None else None
     dev_ms = sum(a.elapsed_time(b) for a, b in step_ev)
@@ -909,6 +930,8 @@ def main():
     ap.add_argument("--spatial-steps", type=int, default=8)
     ap.add_argument("--md", action="store_true", help="also time the device-resident MD step (rows f1+f2); not part of the metric")
     ap.add_argument("--no-graph", action="store_true", help="time eager model(inputs) calls (value and e2e) instead of CUDA-graph replays")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0; cfg5: its owned atoms) as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -924,7 +947,7 @@ def main():
     real_stdout = os.dup(1)
     os.dup2(2, 1)
     if args.config == "cfg5":
-        line = run_spatial(args, rank, world, local_rank)
+        line = run_spatial(args, rank, world, local_rank, dump_dir=args.dump_outputs)
     else:
         line = run_cuda(args, rank, world, local_rank)
         if not args.no_spatial:

@@ -49,6 +49,16 @@ def rel_err(a, b):
     return float(np.max(np.abs(a - b)) / max(np.max(np.abs(b)), 1e-30))
 
 
+def flat_sample(a, k=1024):
+    """A fixed sample of at most ``k`` elements of ``a`` (flattened; every element when there are no more than ``k``).
+    Recorded reference outputs too large to store whole are kept as this sample plus their max-norm, so that a test can
+    still form the ``rel_err`` of the full array's scale.  ``RandomState`` keeps its stream fixed across numpy versions."""
+    a = np.asarray(a).reshape(-1)
+    if a.size <= k:
+        return a
+    return a[np.sort(np.random.RandomState(a.size).choice(a.size, k, replace=False))]
+
+
 @pytest.fixture(scope="session")
 def primitives():
     return np.load(os.path.join(GOLDEN, "primitives.npz"))
